@@ -381,6 +381,24 @@ def envmap_metric(ctx, with_parity=True):
     return res
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_film(out_dir, film):
+    """The (H, W, 5) film a caller of the render receives, as out_dir/film.npy.  A film above DUMP_BYTES (2048^2 of c5) is written as
+    film_sample.npy instead: the (n, 5) rows of a fixed seeded choice of half the budget's worth of pixels, in raster order, the same for
+    every run at that size."""
+    os.makedirs(out_dir, exist_ok=True)
+    film = np.ascontiguousarray(film, np.float32)
+    if film.nbytes <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, "film.npy"), film)
+        return
+    flat = film.reshape(-1, film.shape[-1])
+    n = DUMP_BYTES // 2 // flat[0].nbytes
+    idx = np.sort(np.random.default_rng(0).choice(len(flat), n, replace=False))
+    np.save(os.path.join(out_dir, "film_sample.npy"), flat[idx])
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -398,6 +416,9 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the c3 / c4 / c5 side measurements")
     ap.add_argument("--no-volpath", action="store_true", help="(kept for scripts) same as --no-configs")
     ap.add_argument("--no-traversal", action="store_true", help="skip the isolated BVH-traversal measurement (10 M triangles)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the film of the last timed headline step to DIR/film.npy (float32, H x W x 5; above 64 MB a seeded sample of "
+                         "its pixels, DIR/film_sample.npy) for output-for-output comparisons")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -515,6 +536,8 @@ def main():
     value = samples_per_step / (ms_step / 1e3) / 1e6
     pool = scene.stats()["pool_size"]
     film_host = film.cpu().numpy() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_film(args.dump_outputs, film_host)
 
     # ---- e2e: through the C-ABI with host buffers (scene commit + render into a host film), same metric, same number of steps ----
     host_film = torch.zeros((H, W, 5), dtype=torch.float32).pin_memory()   # the step's result is read back into pinned host memory

@@ -348,8 +348,128 @@ def path_ref_tex():
     print("path_ref_tex.npz:", n, "images")
 
 
+RESAMPLE_UNSEEN = (((48, 40, 3), "mirror", "repeat"), ((9, 31, 1), "zero", "clamp"), ((64, 3, 3), "one", "mirror"))
+MIPMAP_UNSEEN = (("ewa", "repeat", "mirror", 12.0), ("trilinear", "clamp", "zero", 1.0), ("ewa", "one", "clamp", 3.0))
+HALF_UNSEEN = dict(seed=9, n=1_000_000)
+BSDF_NOT_BIT_EXACT = ("plastic", "twosided_two")   # the last bit of one constructor constant (tests/test_oracle_reference_pins.py)
+
+
+def unseen_ref():
+    """The reference's answers on inputs the fixtures above do not hold, for the oracle's tests to compare against.  Outputs are kept as
+    arrays (unseen_ref.npz), except the large ones compared bit for bit -- core, bsdf, instances, <env>, mipmap, half -- which are kept
+    as ref_pins.digest (unseen_ref.json) to keep the fixture small.
+      core/*          core math (ref_pins.run) on ref_pins.inputs(seed=99); fresnel_diffuse_reflectance: util.cpp (fast = false) at FDR_ETAS
+      bsdf/*          the BSDF plugins on ref_pins.bsdf_inputs(seed=4321) (arrays for BSDF_NOT_BIT_EXACT)
+      render/*        partials / filters / ImageBlock::put / Sobol' stream on ref_pins.render_inputs(seed=55)
+      <case>/film     films of ref_pins.unseen_image_cases() (+ <case>/s2c, the reference's sampleToCamera)
+      bitmap/<env>    the environment image the plugin reads back (Emitter::getBitmap, level 0) for ENVMAP_PROBE_CASES
+      conductor_presets/*  every material of data/ior through the reference's spectrum code
+      emitter/sample, instances/*  Scene::sampleEmitterDirect / rayIntersect (instanced) on ref_pins.emitter_probe_inputs()
+      <env>/*         evalEnvironment / pdfEmitterDirect / sampleEmitterDirect of the environment map on ref_pins.envmap_probe_inputs()
+      resample<i>/*, mipmap<i>/*  reference resampler pyramids (RESAMPLE_UNSEEN, seed 77, stored as half) and TMIPMap look-ups (MIPMAP_UNSEEN, seed 99)
+      half            the half rounding of half_inputs(**HALF_UNSEEN)"""
+    sys.path.insert(0, HERE)
+    sys.path.insert(0, os.path.join(HERE, ".."))
+    import dataclasses
+    import ref_pins
+    from bsdf_configs import configs
+    from mitsuba_b200.scene import checker_image
+    from oracle import oracle_api as O
+    ref = lambda name: C.CDLL(os.path.join(HERE, "..", "oracle", "_ref", name))
+    f, digest = ref_pins._f, ref_pins.digest
+    dig, arr = {}, {}
+
+    lib = ref("libcoreref.so")
+    dig.update({"core/" + k: digest(v) for k, v in ref_pins.run(lib, "coreref_", ref_pins.inputs(seed=99)).items()})
+    lib.coreref_fresnel_diffuse_reflectance.restype = C.c_float
+    dig["fresnel_diffuse_reflectance"] = [float(lib.coreref_fresnel_diffuse_reflectance(C.c_float(eta), 0)).hex() for eta in ref_pins.FDR_ETAS]
+
+    lib, x = ref("libbsdfref.so"), ref_pins.bsdf_inputs(seed=4321)
+    for name, b in configs().items():
+        for k, v in ref_pins.run_bsdf_reference(lib, b, x).items():
+            if name in BSDF_NOT_BIT_EXACT:
+                arr[f"bsdf/{name}/{k}"] = v
+            else:
+                dig[f"bsdf/{name}/{k}"] = digest(v)
+
+    arr.update({"render/" + k: v for k, v in ref_pins.run_render(ref("librenderref.so"), "renderref_", ref_pins.render_inputs(seed=55)).items()})
+
+    lib = ref("libpathref.so")
+    for name, desc, rp in ref_pins.unseen_image_cases():
+        arr[name + "/film"], arr[name + "/s2c"] = ref_pins.reference_render(lib, desc, rp, want_camera=True)
+    env_cases = {name: (desc, rp) for name, desc, rp in ref_pins.image_cases_env()}
+    for name in ref_pins.ENVMAP_PROBE_CASES:
+        h = ref_pins.reference_scene(lib, *env_cases[name])
+        wh = (C.c_int * 2)()
+        assert lib.pathref_environment_bitmap(h, wh, None) == 0
+        bitmap = np.zeros((wh[1], wh[0], 3), np.float32)
+        assert lib.pathref_environment_bitmap(h, wh, f(bitmap)) == 0
+        arr["bitmap/" + name] = bitmap
+    names, values = [], []
+    for line in open(os.path.join(HERE, "..", "mitsuba_b200", "data", "conductor_presets.txt")):
+        t = line.split()
+        if t and not t[0].startswith("#"):
+            e, kk = np.zeros(3, np.float32), np.zeros(3, np.float32)
+            assert lib.pathref_conductor_preset(os.path.join(REF, "data").encode(), t[0].encode(), f(e), f(kk)) == 0
+            names.append(t[0]); values.append(np.concatenate([e, kk]))
+    arr["conductor_presets/names"], arr["conductor_presets/eta_k"] = np.array(names), np.stack(values)
+
+    refp, smp, pos = ref_pins.emitter_probe_inputs()
+    cases = {name: (desc, rp) for name, desc, rp in ref_pins.image_cases_ext()}
+    h = ref_pins.reference_scene(lib, *cases["env_plus_area_cbox"])
+    a = np.zeros((len(refp), 12), np.float32)
+    lib.pathref_sample_emitter_direct(h, len(refp), f(refp), f(smp), f(a))
+    arr["emitter/sample"] = a
+    desc, rp = cases["instances_sobol"]
+    h = ref_pins.reference_scene(lib, desc, rp)
+    arr["instances/s2c"] = np.zeros((4, 4), np.float32)
+    lib.pathref_sample_to_camera(h, f(arr["instances/s2c"]))
+    arr["instances/inverses"] = np.stack(ref_pins.reference_instance_inverses(lib, desc))
+    rays = O.OracleScene(desc, sample_to_camera=arr["instances/s2c"], instance_inverses=list(arr["instances/inverses"])).camera_rays(pos)
+    a = np.zeros((len(pos), 24), np.float32)
+    lib.pathref_intersect(h, len(pos), f(rays), f(a))
+    dig.update({"instances/" + k: digest(v) for k, v in ref_pins.intersection_views(a).items()})
+    for name, rays, rd, refp, dd, smp in ref_pins.envmap_probe_inputs():
+        desc, rp = env_cases[name]
+        inv = ref_pins.reference_envmap_inverse(lib, desc)
+        if inv is not None:
+            desc.envmap = dataclasses.replace(desc.envmap, to_local=inv)
+            arr[name + "/to_local"] = inv
+        h = ref_pins.reference_scene(lib, desc, rp)
+        n = len(rays)
+        ev, evd, pdf, s = np.zeros((n, 3), np.float32), np.zeros((n, 3), np.float32), np.zeros(n, np.float32), np.zeros((n, 12), np.float32)
+        lib.pathref_eval_environment(h, n, 0, f(rays), f(ev))
+        lib.pathref_eval_environment(h, n, 1, f(rd), f(evd))
+        lib.pathref_pdf_environment_direct(h, n, f(refp), f(dd), f(pdf))
+        lib.pathref_sample_emitter_direct(h, n, f(refp), f(smp), f(s))
+        dig.update({name + "/eval": digest(ev), name + "/eval_diff": digest(evd), name + "/pdf": digest(pdf)})
+        dig.update({f"{name}/sample_{k}": digest(v) for k, v in ref_pins.emitter_sample_views(s).items()})
+
+    lib, rng = ref("librfilterref.so"), np.random.default_rng(77)
+    for i, (shape, wu, wv) in enumerate(RESAMPLE_UNSEEN):
+        img = np.maximum((rng.random(shape) * 1.2 - 0.05).astype(np.float32), 0)
+        for l, lvl in enumerate(reference_pyramid(img, wu, wv, lib)):
+            arr[f"resample{i}/{l + 1}"] = half_store(lvl)
+    rng, img = np.random.default_rng(99), checker_image(70, 45, 6, 1)
+    for i, (ft, wu, wv, aniso) in enumerate(MIPMAP_UNSEEN):
+        m = ReferenceMipmap([img] + reference_pyramid(img, wu, wv), wu, wv, ft, aniso)
+        uv, pt = texture_lookups(rng, 20000)
+        dig[f"mipmap{i}/filtered"], dig[f"mipmap{i}/unfiltered"] = digest(m.eval(uv, pt)), digest(m.eval(uv))
+    x = half_inputs(**HALF_UNSEEN)
+    y = np.zeros_like(x)
+    ref("libcoreref.so").coreref_half_round(len(x), f(x), f(y))
+    dig["half"] = digest(y.view(np.uint32))   # the bits: the sign of zero included
+
+    json.dump(dig, open(os.path.join(OUT, "unseen_ref.json"), "w"), indent=0, sort_keys=True)
+    np.savez_compressed(os.path.join(OUT, "unseen_ref.npz"), **arr)
+    print("unseen_ref.json:", len(dig), "digests; unseen_ref.npz:", len(arr), "arrays")
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
+    if "--unseen-only" in sys.argv:
+        unseen_ref()
+        sys.exit(0)
     if "--tex-only" in sys.argv:
         path_ref_tex()
         sys.exit(0)
@@ -379,3 +499,4 @@ if __name__ == "__main__":
     resample_ref()
     half_ref()
     mipmap_ref()
+    unseen_ref()

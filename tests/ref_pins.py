@@ -655,3 +655,73 @@ def image_cases_tex():
     d.meshes[3].bsdf = Bsdf("roughconductor", distribution="ggx", alpha_u=0.3, alpha_v=0.3, eta=(0.2004, 0.9240, 1.1022), k=(3.9129, 2.4528, 2.1421),
                             specular_reflectance=d.meshes[3].bsdf.reflectance)
     yield "tex_plastic_and_conductor", d, RenderParams(spp=8, sampler="sobol", rfilter="gaussian")
+
+
+# ---------------------------------------------------------------------------------------------------------------------------
+# inputs the fixtures above do not hold: tests/gen_golden.py (unseen_ref) stores the reference's answers to them in
+# tests/golden/unseen_ref.{json,npz}, and tests/test_oracle_*.py hold the oracle to them
+# ---------------------------------------------------------------------------------------------------------------------------
+FDR_ETAS = (1.5, 1.0 / 1.5, 1.33, 1.49)
+ENVMAP_PROBE_CASES = ("envmap_only_ball", "envmap_plus_area_cbox")
+
+
+def digest(a):
+    """SHA-256 of an array's dtype, shape and values, with every NaN one NaN and -0 as +0 (the equality `same` of the tests checks): what
+    the unseen-input fixture keeps of a large output that is compared bit for bit, instead of the array.  Hash an integer view to keep
+    the sign of zero and the NaN payloads."""
+    import hashlib
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        a = np.ascontiguousarray(np.where(np.isnan(a), a.dtype.type(np.nan), a + a.dtype.type(0)))
+    return hashlib.sha256(repr((a.dtype.str, a.shape)).encode() + a.tobytes()).hexdigest()
+
+
+def emitter_sample_views(a):
+    """The parts of Scene::sampleEmitterDirect records (n, 12) that are compared: the success flag of every record, whole successful records."""
+    ok = a[:, 8] == 1
+    return {"flag": a[:, 8], "ok_rows": a[ok]}
+
+
+def intersection_views(a):
+    """The parts of Scene::rayIntersect records (n, 24) that are compared: the hit flag of every ray, columns 0-18 and 20 of the hits."""
+    hit = a[:, 21] == 1
+    return {"hit": a[:, 21], "hit_cols": a[hit][:, :19], "hit_col20": a[hit, 20]}
+
+
+def unseen_image_cases():
+    """Two more films of the assembled reference renderer: a Cornell box and a textured scene with mirror wrapping."""
+    from mitsuba_b200.scene import RenderParams, cornell_box, textured_scene
+    yield "cbox_56x40", cornell_box(56, 40), RenderParams(spp=12, sampler="sobol", rfilter="gaussian", seed=3)
+    yield "textured_mirror", textured_scene(44, 36, filter_type="ewa", tex_res=48, wrap="mirror", n_theta=10, n_phi=20), \
+        RenderParams(spp=6, sampler="sobol", rfilter="gaussian", seed=5)
+
+
+def emitter_probe_inputs():
+    """Reference points / selection samples for Scene::sampleEmitterDirect (400) and film positions of camera rays into the instanced
+    scene (3000)."""
+    rng = np.random.default_rng(99)
+    n = 400
+    refp = np.zeros((n, 6), np.float32)
+    refp[:, 0:3] = rng.uniform(50, 500, (n, 3)); refp[:, 3:6] = _dirs(rng, n)
+    smp = rng.random((n, 2)).astype(np.float32)
+    pos = (rng.random((3000, 2)) * 40).astype(np.float32)
+    return refp, smp, pos
+
+
+def envmap_probe_inputs(n=3000):
+    """Per case of ENVMAP_PROBE_CASES: directions (poles and the seam first), the same with ray differentials from a fraction of a texel
+    to strongly anisotropic footprints, reference points + directions for the direct-sampling density, and direct-sampling samples."""
+    rng = np.random.default_rng(5)
+    for name in ENVMAP_PROBE_CASES:
+        rays = np.zeros((n, 6), np.float32); rays[:, 3:] = _dirs(rng, n)
+        rays[:3, 3:] = [(0, 1, 0), (0, -1, 0), (0, 0, 1)]
+        rd = np.zeros((n, 18), np.float32); rd[:, :6] = rays
+        for k, sc in ((9, 0.02), (15, 0.3)):
+            v = rays[:, 3:] + sc * rng.standard_normal((n, 3)).astype(np.float32) * rng.random((n, 1)).astype(np.float32) ** 2
+            rd[:, k:k + 3] = v / np.linalg.norm(v, axis=1, keepdims=True)
+        refp = np.zeros((n, 6), np.float32)
+        refp[:, 0:3] = rng.uniform(-1, 1, (n, 3)) if name == "envmap_only_ball" else rng.uniform(50, 500, (n, 3))
+        refp[:, 3:6] = _dirs(rng, n)
+        dd = _dirs(rng, n).astype(np.float32)
+        smp = rng.random((n, 2)).astype(np.float32)
+        yield name, rays, rd, refp, dd, smp

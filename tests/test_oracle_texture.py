@@ -4,6 +4,7 @@ The reference holds no golden vectors for mipmap.h / bitmap.cpp, so the restatem
 unity, known-answer weights from an independent float64 derivation, analytic uv derivatives of a plane) and by a second,
 independently written implementation (the host-side pyramid builder that feeds the device)."""
 import ctypes as C
+import json
 import math
 import os
 
@@ -280,20 +281,25 @@ def test_pyramids_match_the_reference_resampler():
         assert f"lvl{k}_{info['levels']}" not in g.files  # same number of levels
 
 
+# the reference's outputs on inputs the fixtures above do not hold (tests/gen_golden.py, unseen_ref): the `*_when_present` tests below
+# compare with these stored outputs and do not call the reference's libraries
+UNSEEN = json.load(open(os.path.join(os.path.dirname(GOLDEN), "unseen_ref.json")))
+UNSEEN_ARRAYS = np.load(os.path.join(os.path.dirname(GOLDEN), "unseen_ref.npz"))
+
+
 def test_live_reference_resampler_when_present():
-    """Same comparison against the freshly compiled reference code (only where oracle/_ref/librfilterref.so exists)."""
-    so = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "oracle", "_ref", "librfilterref.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref/librfilterref.so not built (the reference tree is not on this machine)")
-    from gen_golden import half_store, reference_pyramid
-    lib = C.CDLL(so)
+    """Same comparison on images the fixture does not hold: the levels the reference resampler (oracle/_ref/librfilterref.so) made of them,
+    stored as half, in tests/golden/unseen_ref.npz."""
+    from gen_golden import RESAMPLE_UNSEEN, half_store
     rng = np.random.default_rng(77)
-    for shape, wu, wv in (((48, 40, 3), "mirror", "repeat"), ((9, 31, 1), "zero", "clamp"), ((64, 3, 3), "one", "mirror")):
+    for i, (shape, wu, wv) in enumerate(RESAMPLE_UNSEEN):
         img = np.maximum((rng.random(shape) * 1.2 - 0.05).astype(np.float32), 0)
         tex = Texture(img if shape[2] == 3 else img[:, :, 0], filter_type="trilinear", wrap_u=wu, wrap_v=wv)
         sc = O.OracleScene(one_texture_scene(tex))
-        for l, ref in enumerate(reference_pyramid(img, wu, wv, lib)):
-            assert np.array_equal(sc.texture_level(0, l + 1), half_store(ref))
+        levels = [UNSEEN_ARRAYS[f"resample{i}/{l}"] for l in range(1, sc.texture_info(0)["levels"])]
+        assert f"resample{i}/{len(levels) + 1}" not in UNSEEN_ARRAYS.files  # same number of levels
+        for l, ref in enumerate(levels):
+            assert np.array_equal(sc.texture_level(0, l + 1), ref), (i, l + 1)
         assert np.array_equal(sc.texture_level(0, 0), half_store(img if shape[2] == 3 else img[:, :, :1]).reshape(sc.texture_level(0, 0).shape))
 
 
@@ -319,19 +325,18 @@ def test_lookups_match_the_reference_mipmap():
 
 
 def test_live_reference_mipmap_when_present():
-    so = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "oracle", "_ref", "libmipmapref.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref/libmipmapref.so not built (the reference tree is not on this machine)")
-    from gen_golden import ReferenceMipmap, reference_pyramid, texture_lookups
+    """Look-ups on a checkerboard the fixture does not hold, against the digests of what the reference's TMIPMap (oracle/_ref/libmipmapref.so)
+    returns over the reference resampler's pyramid (tests/golden/unseen_ref.json)."""
+    from gen_golden import MIPMAP_UNSEEN, texture_lookups
+    from ref_pins import digest
     rng = np.random.default_rng(99)
     img = checker_image(70, 45, 6, 1)
-    for ft, wu, wv, aniso in (("ewa", "repeat", "mirror", 12.0), ("trilinear", "clamp", "zero", 1.0), ("ewa", "one", "clamp", 3.0)):
+    for i, (ft, wu, wv, aniso) in enumerate(MIPMAP_UNSEEN):
         tex = Texture(img, filter_type=ft, wrap_u=wu, wrap_v=wv, max_anisotropy=aniso)
         sc = O.OracleScene(one_texture_scene(tex))
-        ref = ReferenceMipmap([img] + reference_pyramid(img, wu, wv), wu, wv, ft, aniso)
         uv, pt = texture_lookups(rng, 20000)
-        assert np.array_equal(sc.texture_eval(0, uv, pt), ref.eval(uv, pt))
-        assert np.array_equal(sc.texture_eval(0, uv), ref.eval(uv))
+        assert digest(sc.texture_eval(0, uv, pt)) == UNSEEN[f"mipmap{i}/filtered"]
+        assert digest(sc.texture_eval(0, uv)) == UNSEEN[f"mipmap{i}/unfiltered"]
 
 
 def test_half_storage_rounding_matches_the_reference_half_class():
@@ -347,14 +352,13 @@ def test_half_storage_rounding_matches_the_reference_half_class():
     O.lib().orc_half_round(C.c_uint64(len(x)), x.ctypes.data_as(C.POINTER(C.c_float)), out.ctypes.data_as(C.POINTER(C.c_float)))
     assert np.array_equal(out.view(np.uint32), y.view(np.uint32))
     assert np.array_equal(half_store(x).view(np.uint32), y.view(np.uint32))
-    so = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "oracle", "_ref", "libcoreref.so")
-    if os.path.exists(so):   # live: two million fresh values
-        lib = C.CDLL(so)
-        x = half_inputs(seed=9, n=1_000_000)
-        ref, out = np.zeros_like(x), np.zeros_like(x)
-        lib.coreref_half_round(len(x), x.ctypes.data_as(C.POINTER(C.c_float)), ref.ctypes.data_as(C.POINTER(C.c_float)))
-        O.lib().orc_half_round(C.c_uint64(len(x)), x.ctypes.data_as(C.POINTER(C.c_float)), out.ctypes.data_as(C.POINTER(C.c_float)))
-        assert np.array_equal(out.view(np.uint32), ref.view(np.uint32)) and np.array_equal(half_store(x).view(np.uint32), ref.view(np.uint32))
+    # three million fresh values: oracle and numpy agree on all of them, and with the reference (digest of the bits in tests/golden/unseen_ref.json)
+    from gen_golden import HALF_UNSEEN
+    from ref_pins import digest
+    x = half_inputs(**HALF_UNSEEN)
+    out = np.zeros_like(x)
+    O.lib().orc_half_round(C.c_uint64(len(x)), x.ctypes.data_as(C.POINTER(C.c_float)), out.ctypes.data_as(C.POINTER(C.c_float)))
+    assert np.array_equal(half_store(x).view(np.uint32), out.view(np.uint32)) and digest(out.view(np.uint32)) == UNSEEN["half"]
 
 
 def test_stored_texels_are_half_representable_and_the_maximum_is_not():
